@@ -53,6 +53,8 @@ SEED = 1234 + 3
 WORKLOAD = '3840x2160 Q50 4:4:4 synthetic JPEG coefficients, joint 3 planes, -i 100 -w 0.3 -p 0.001'
 METRIC = 'Mpixel-iterations/s'
 FALLBACK_HBM_GBS = 6650.0
+DUMP_BYTES = 64 * 10**6          # --dump-outputs writes at most this much in all
+DUMP_SEED = 20240601
 
 
 def algorithmic_bytes(img, nchannel=3):
@@ -145,6 +147,23 @@ def emit(line, world):
     print(text, flush=True)
     if world > 1:
         print(text, file=sys.stderr, flush=True)
+
+
+def dump_outputs(directory, arrays):
+    """Write each float32 array as DIR/<name>.npy.  When they are larger than DUMP_BYTES together,
+    each is replaced by the same fixed, seeded sample of its flattened elements (positions sorted),
+    so two runs with the same arguments write files that compare element for element."""
+    os.makedirs(directory, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(v, np.float32) for k, v in arrays.items()}
+    header = 128                                  # .npy header of a 1-D or 2-D float32 array
+    if sum(a.nbytes + header for a in arrays.values()) > DUMP_BYTES:
+        keep = (DUMP_BYTES // len(arrays) - header) // 4
+        for k, a in arrays.items():
+            idx = np.sort(np.random.default_rng(DUMP_SEED).choice(a.size, size=min(keep, a.size), replace=False))
+            arrays[k] = a.reshape(-1)[idx]
+        print(f'bench.py: outputs sampled to {keep} of their elements each (seed {DUMP_SEED})', file=sys.stderr, flush=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(directory, f'{k}.npy'), a)
 
 
 def make_frame(seed):
@@ -248,8 +267,11 @@ def run_reference_arm(args, rank, world):
     for _ in range(args.warmup):
         cpu_solve_rate(img, fdata, it, kind)
     dt = 0.0
-    for _ in range(args.steps):
-        dt += cpu_solve_rate(img, fdata, it, kind)[1]
+    planes = []
+    for k in range(args.steps):
+        dt += cpu_solve_rate(img, fdata, it, kind, keep=planes if k == args.steps - 1 else None)[1]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {f'plane{c}': p for c, p in enumerate(planes)})
     value = img.width * img.height * it * args.steps / dt / 1e6
     sample = f'{WIDTH}x{HEIGHT} 4:4:4 frame, {it} of {ITERATIONS} iterations per step (per-iteration cost is iteration-count independent)'
     line = {
@@ -340,6 +362,14 @@ def run_product_arm(args, rank, local_rank, world):
     barrier()
     ms_total = max_over_ranks(ev0.elapsed_time(ev1))
     launches = int(lib.j2p_session_launches(s) - launches0)
+    if args.dump_outputs and rank == 0:
+        # the three frame planes the last timed solve left in HBM, before anything else runs on the session
+        planes = {}
+        for c in range(3):
+            planes[f'plane{c}'] = np.empty((H, W), np.float32)
+            if lib.j2p_session_download(s, c, planes[f'plane{c}'].ctypes.data) != 0:
+                raise RuntimeError(lib.j2p_last_error().decode())
+        dump_outputs(args.dump_outputs, planes)
 
     # ---- per-kernel live timing for the roofline (rank 0, N=1 semantics: one GPU's kernels) ----
     mg, mp = C.c_float(), C.c_float()
@@ -611,7 +641,12 @@ def main():
     ap.add_argument('--steps', type=int, default=5)
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write the planes the last step computed as DIR/<name>.npy '
+                         f'(float32; a fixed seeded sample when larger than {DUMP_BYTES // 10**6} MB in all)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     rank = int(os.environ.get('RANK', '0'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))

@@ -122,6 +122,19 @@ def run_compute(kind: str, img: CoefImage, channels, weight, pweight, iterations
     return (out, log) if want_log else out
 
 
+def transform8x8(fn, block) -> np.ndarray:
+    """Apply an in-place 8x8 transform (dct8x8s / idct8x8s and their restatements) to a copy of block."""
+    p = abi.alloc_floats(64)
+    try:
+        C.memmove(p, np.ascontiguousarray(block, np.float32).ctypes.data, 256)
+        fn(p)
+        out = np.empty(64, np.float32)
+        C.memmove(out.ctypes.data, p, 256)
+    finally:
+        abi.free_ptr(p)
+    return out
+
+
 def bits(a: np.ndarray) -> np.ndarray:
     return np.ascontiguousarray(a, dtype=np.float32).view(np.uint32)
 

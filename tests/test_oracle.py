@@ -1,7 +1,6 @@
-"""CPU tests: the oracle restatement against the golden vectors and (when it is present) against
-the compiled reference itself.  Bit-exact everywhere: the path is fp32/fp64 arithmetic in a fixed
-IEEE operation order, so "equal" means equal bit patterns."""
-import ctypes as C
+"""CPU tests: the oracle restatement against the golden vectors and against recorded runs of the
+original jpeg2png (tests/golden/reference_runs.npz).  Bit-exact everywhere: the path is fp32/fp64
+arithmetic in a fixed IEEE operation order, so "equal" means equal bit patterns."""
 import os
 
 import numpy as np
@@ -9,7 +8,8 @@ import pytest
 
 from jpeg2png_b200 import synth
 from tests import helpers as H
-from tests.golden_io import golden_cases, load_case
+from tests.golden_io import (assert_matches_recorded, block_crc, golden_cases, load_case, load_reference_run,
+                             load_reference_transforms)
 
 needs_ref = pytest.mark.skipif(not (H.have_ref() or os.path.exists(H.REFERENCE_SRC)),
                                reason='compiled reference (oracle/_ref) not available on this machine')
@@ -44,64 +44,48 @@ def test_reference_reproduces_golden(name):
     H.assert_bit_identical(out, g['out'], f'ref {name}')
 
 
-@needs_ref
 def test_reference_simd_equals_scalar():
-    """The reference's own invariant (compute_simd_step.c:103-104, :223-224)."""
-    img = synth.synth_coefs(96, 64, 10, '4:2:0', 11)
-    f = H.decode_planes(img)
-    a = H.run_compute('ref', img, [0, 1, 2], 0.3, [0.001] * 3, 25, f)
-    b = H.run_compute('ref_c', img, [0, 1, 2], 0.3, [0.001] * 3, 25, f)
-    H.assert_bit_identical(a, b, 'simd vs c')
+    """The reference's own invariant (compute_simd_step.c:103-104, :223-224): its SIMD and scalar
+    builds were recorded on the same frame; the restatement must reproduce both bit for bit."""
+    run = load_reference_run('simd_vs_scalar')
+    out = H.run_compute('oracle', run['img'], run['channels'], run['weight'], run['pweight'], run['iterations'])
+    assert_matches_recorded(out, run['out'], 'oracle vs reference SIMD build')
+    assert_matches_recorded(out, run['scalar_out'], 'oracle vs reference scalar build')
 
 
-@needs_ref
-@pytest.mark.parametrize('w,h,q,ss,channels,weight,pw,iters', [
+# (w, h, quality, subsampling, channels, weight, pweights, iterations); the frames were synthesised
+# with seed 1234 + w + h and the original's outputs recorded by tests/golden/make_reference_runs.py
+REFERENCE_CONFIGS = [
     (256, 256, 10, '4:2:0', [0, 1, 2], 0.3, [0.001] * 3, 50),      # BASELINE config 1
     (256, 256, 10, '4:2:0', [2], 0.3, [0.001], 50),                # config 1, separate mode, chroma
     (200, 120, 30, '4:2:0', [0, 1, 2], 0.3, [0.001] * 3, 30),      # luma grid narrower/shorter than the frame
     (136, 72, 50, '4:4:4', [0, 1, 2], 0.7, [0.001, 0.0, 0.01], 40),
     (64, 64, 90, '4:4:4', [0, 1, 2], 0.0, [0.0] * 3, 20),          # TV only
-])
+]
+
+
+@pytest.mark.parametrize('w,h,q,ss,channels,weight,pw,iters', REFERENCE_CONFIGS)
 def test_oracle_matches_reference(w, h, q, ss, channels, weight, pw, iters):
-    img = synth.synth_coefs(w, h, q, ss, seed=1234 + w + h)
-    f = H.decode_planes(img, channels)
-    ref = H.run_compute('ref', img, channels, weight, pw, iters, f)
-    ora = H.run_compute('oracle', img, channels, weight, pw, iters, f)
-    H.assert_bit_identical(ref, ora, 'ref vs oracle')
+    run = load_reference_run(f'config{REFERENCE_CONFIGS.index((w, h, q, ss, channels, weight, pw, iters))}')
+    assert (run['img'].width, run['img'].height, run['channels'], run['iterations']) == (w, h, channels, iters)
+    ora = H.run_compute('oracle', run['img'], channels, weight, pw, iters)
+    assert_matches_recorded(ora, run['out'], 'ref vs oracle')
 
 
-@needs_ref
 def test_oracle_matches_reference_random_planes():
     for seed in range(5):
-        img = synth.random_coefs([(40, 24), (24, 16), (16, 8)], [(1, 1), (2, 2), (3, 4)], seed)
-        f = H.decode_planes(img)
-        ref = H.run_compute('ref', img, [0, 1, 2], 0.4, [0.001] * 3, 12, f)
-        ora = H.run_compute('oracle', img, [0, 1, 2], 0.4, [0.001] * 3, 12, f)
-        H.assert_bit_identical(ref, ora, f'random seed {seed}')
+        run = load_reference_run(f'random_planes{seed}')
+        ora = H.run_compute('oracle', run['img'], [0, 1, 2], 0.4, [0.001] * 3, 12)
+        assert_matches_recorded(ora, run['out'], f'random seed {seed}')
 
 
-@needs_ref
 def test_transforms_match_reference():
-    """8x8 DCT / IDCT restatement vs ooura/dct.c on random and extreme blocks."""
-    ref, ora = H.load_ref(), H.load_oracle()
-    rng = np.random.default_rng(5)
-    blocks = [rng.normal(0, s, 64).astype(np.float32) for s in (1e-3, 1.0, 50.0, 1e4, 1e-30) for _ in range(40)]
-    blocks += [np.zeros(64, np.float32), np.full(64, 127.5, np.float32), -np.ones(64, np.float32) * 1e-42]
-    for b in blocks:
-        for fr, fo in ((ref.dct8x8s, ora.oracle_dct8x8), (ref.idct8x8s, ora.oracle_idct8x8)):
-            a = np.array(b, dtype=np.float32)
-            c = np.array(b, dtype=np.float32)
-            pa = H.abi.alloc_floats(64)
-            pc = H.abi.alloc_floats(64)
-            C.memmove(pa, a.ctypes.data, 256)
-            C.memmove(pc, c.ctypes.data, 256)
-            fr(pa)
-            fo(pc)
-            C.memmove(a.ctypes.data, pa, 256)
-            C.memmove(c.ctypes.data, pc, 256)
-            H.abi.free_ptr(pa)
-            H.abi.free_ptr(pc)
-            assert (H.bits(a) == H.bits(c)).all()
+    """8x8 DCT / IDCT restatement vs ooura/dct.c on random and extreme blocks (denormals included)."""
+    ora = H.load_oracle()
+    blocks, want_dct, want_idct = load_reference_transforms()
+    for i, (b, wd, wi) in enumerate(zip(blocks, want_dct, want_idct)):
+        assert block_crc(H.transform8x8(ora.oracle_dct8x8, b)) == wd, f'DCT of block {i}'
+        assert block_crc(H.transform8x8(ora.oracle_idct8x8, b)) == wi, f'IDCT of block {i}'
 
 
 def test_oracle_objective_log_decreases():
@@ -132,29 +116,14 @@ def test_rgb_conversion_restatement():
     assert (int(v[1, 0, 0]) << 8 | int(v[1, 0, 1])) == 255 * 256
 
 
-@needs_ref
 @pytest.mark.parametrize('seed', range(16))
 def test_oracle_matches_reference_random_sweep(seed):
     """Randomised configurations (plane sizes, sampling factors up to 3x4, zero and non-zero weights,
-    single-plane and joint mode, planes smaller than the frame): restatement == compiled reference."""
-    rng = np.random.default_rng(1000 + seed)
-    nplanes = 3
-    samp = [(1, 1)] + [(int(rng.integers(1, 4)), int(rng.integers(1, 5))) for _ in range(2)]
-    fw, fh = 8 * int(rng.integers(2, 9)), 8 * int(rng.integers(2, 7))
-    dims = []
-    for (sw, sh) in samp:
-        cw, ch = -(-fw // sw), -(-fh // sh)
-        cw, ch = -(-cw // 8) * 8, -(-ch // 8) * 8
-        if rng.random() < 0.3 and cw > 8:
-            cw -= 8                                               # a plane that does not cover the frame
-        dims.append((cw, ch))
-    img = synth.random_coefs(dims, samp, seed=seed, amplitude=int(rng.integers(5, 60)), qmax=int(rng.integers(2, 80)))
-    joint = rng.random() < 0.6
-    channels = [0, 1, 2] if joint else [int(rng.integers(0, nplanes))]
-    weight = float(rng.choice([0.0, 0.1, 0.3, 1.0]))
-    pw = [float(rng.choice([0.0, 0.001, 0.05])) for _ in channels]
-    iters = int(rng.integers(1, 25))
-    f = H.decode_planes(img, channels)
-    a = H.run_compute('ref', img, channels, weight, pw, iters, [p.copy() for p in f])
-    b = H.run_compute('oracle', img, channels, weight, pw, iters, [p.copy() for p in f])
-    H.assert_bit_identical(b, a, f'sweep seed {seed}: samp {samp} dims {dims} channels {channels} w {weight} p {pw} i {iters}')
+    single-plane and joint mode, planes smaller than the frame; drawn by
+    tests/golden/make_reference_runs.py): restatement == recorded reference."""
+    run = load_reference_run(f'sweep{seed}')
+    img = run['img']
+    b = H.run_compute('oracle', img, run['channels'], run['weight'], run['pweight'], run['iterations'])
+    assert_matches_recorded(b, run['out'], f"sweep seed {seed}: samp {[(p.w_samp, p.h_samp) for p in img.planes]} "
+                                           f"dims {[(p.w, p.h) for p in img.planes]} channels {run['channels']} "
+                                           f"w {run['weight']} p {run['pweight']} i {run['iterations']}")
