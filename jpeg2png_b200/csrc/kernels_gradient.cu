@@ -1,4 +1,5 @@
-// kernels_gradient.cu — sm_100a sub-gradient kernel of the jpeg2png solver.
+// kernels_gradient.cu — sm_100a sub-gradient kernel of the jpeg2png solver, scalar build: it runs
+// for sessions with objective logging (the default path is kernels_gradient_packed.cu).
 //
 // One solver iteration (reference compute.c:427-453) is two kernels:
 //
@@ -48,7 +49,7 @@ namespace j2p {
 // is set to 0, which makes every quotient of that pixel exactly 0.
 // ------------------------------------------------------------------------------------------
 // LOG: additionally sum the objective terms the reference logs (compute.c:91,155: tv += alpha*norm
-// per pixel, fp64) — only instantiated for sessions with logging enabled (-c csv).
+// per pixel, fp64).  Only the LOG = true builds are launched (sessions with logging enabled, -c csv).
 template <int NC, bool LOG, bool TGV>
 __global__ void __launch_bounds__(GM_NT, J2P_GRAD_MIN_CTAS) k_gradient(const __grid_constant__ FrameDev F, const float factor, const int band_rows) {
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -463,51 +464,37 @@ bool pdl_enabled() {
     return on;
 }
 
-// J2P_GRAD_SCALAR=1: the scalar kernel for every session (A/B aid; it is always the -c csv build)
-static bool g_grad_scalar = false;
-
 // once per device and process; *slots = resident CTAs of the gradient kernel on the current device
 cudaError_t configure_kernels(int *slots) {
-    int per_sm = 0, dev = 0, sms = 0;
+    int dev = 0, sms = 0;
     cudaError_t e = configure_project_kernels();
     if (e != cudaSuccess) return e;
     e = cudaGetDevice(&dev);
     if (e != cudaSuccess) return e;
     e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     if (e != cudaSuccess) return e;
-    const char *env = getenv("J2P_GRAD_SCALAR");
-    g_grad_scalar = env && *env == '1';
-    if (g_grad_scalar) {
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_gradient<3, false, true>, GM_NT, 0);
-        if (e != cudaSuccess) return e;
-    } else {
-        per_sm = packed_gradient_occupancy();
-    }
+    const int per_sm = packed_gradient_occupancy();
     *slots = sms * (per_sm > 0 ? per_sm : 1);
     return cudaSuccess;
 }
 
-template <bool LOG, bool TGV>
+template <bool TGV>
 static void launch_gradient_nc(const FrameDev &F, float factor, dim3 grid, int rows, cudaStream_t s) {
     switch (F.nc) {
-        case 1: k_gradient<1, LOG, TGV><<<grid, GM_NT, 0, s>>>(F, factor, rows); break;
-        case 2: k_gradient<2, LOG, TGV><<<grid, GM_NT, 0, s>>>(F, factor, rows); break;
-        default: k_gradient<3, LOG, TGV><<<grid, GM_NT, 0, s>>>(F, factor, rows); break;
+        case 1: k_gradient<1, true, TGV><<<grid, GM_NT, 0, s>>>(F, factor, rows); break;
+        case 2: k_gradient<2, true, TGV><<<grid, GM_NT, 0, s>>>(F, factor, rows); break;
+        default: k_gradient<3, true, TGV><<<grid, GM_NT, 0, s>>>(F, factor, rows); break;
     }
 }
 
 cudaError_t launch_gradient(const FrameDev &F, float factor, cudaStream_t s) {
-    if (!F.log_on && !g_grad_scalar) return launch_gradient_packed(F, factor, s);
+    if (!F.log_on) return launch_gradient_packed(F, factor, s);
+    // objective logging: the scalar kernel, which also sums the TV / TGV terms
     int cx, bands, rows;
     grad_geometry(F.W, F.t1 - F.t0, F.grad_slots, &cx, &bands, &rows);
     const dim3 grid(cx, bands);
-    if (F.log_on) {
-        if (F.use_tgv) launch_gradient_nc<true, true>(F, factor, grid, rows, s);
-        else launch_gradient_nc<true, false>(F, factor, grid, rows, s);
-    } else {
-        if (F.use_tgv) launch_gradient_nc<false, true>(F, factor, grid, rows, s);
-        else launch_gradient_nc<false, false>(F, factor, grid, rows, s);
-    }
+    if (F.use_tgv) launch_gradient_nc<true>(F, factor, grid, rows, s);
+    else launch_gradient_nc<false>(F, factor, grid, rows, s);
     return cudaGetLastError();
 }
 

@@ -1,4 +1,6 @@
-// kernels_project.cu — step + projection kernel, conventional decode, aux_init.
+// kernels_project.cu — the choice of each plane's projection kernel and its launch; the
+// k_project<SW, SH> step + projection kernel (objective logging, odd sampling factors); the step of
+// the pixels no coefficient block covers; conventional decode; aux_init.
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdlib.h>
@@ -12,12 +14,12 @@
 
 namespace j2p {
 
-cudaError_t launch_project_tile(const FrameDev &F, int c, int count, float factor, cudaStream_t s, int *nlaunch, bool uncovered_only);
+cudaError_t launch_project_tile(const FrameDev &F, int c, int count, float factor, cudaStream_t s);
 cudaError_t configure_project_tma();
 bool project_tma_enabled();
 cudaError_t launch_project_tma(const FrameDev &F, const TileMaps &M, int c, int count, int xsel, float factor, cudaStream_t s);
 cudaError_t configure_project_tile22();
-cudaError_t launch_project_tile22(const FrameDev &F, int c, int count, float factor, cudaStream_t s, int *nlaunch);
+cudaError_t launch_project_tile22(const FrameDev &F, int c, int count, float factor, cudaStream_t s);
 
 // ------------------------------------------------------------------------------------------
 // k_project — 8 threads per coefficient block (thread j owns row j), 32 blocks per CTA.
@@ -70,21 +72,9 @@ __global__ void __launch_bounds__(P_NT, (SW * SH <= 1) ? J2P_PROJ_MIN_CTAS : 2) 
             }
         }
     }
-    if (tid < 64) {
-        sq[0][tid] = F.q[c][tid];
-        sq[1][tid] = F.qq[c][tid];
-        sq[2][tid] = F.rqq[c][tid];
-    } else if (tid < 96) {
-        strip_norm(F, c, snorm, tid - 64);                         // whole frame: what k_gradient left; strips: fold of every rank's sums
-    }
+    stage_tables(F, c, &sq[0][0], snorm, tid);
     __syncthreads();
-    Stepper stepper;
-    stepper.factor = factor;
-    stepper.step = F.step;
-    stepper.norm = snorm[0];
-    stepper.rn = snorm[1];
-    stepper.stepping = stepper.norm != 0.f;                        // compute.c:211
-    const bool norm_ok = qdiv_divisor_ok(stepper.norm);
+    const Stepper stepper(factor, F.step, snorm[0], snorm[1]);
     float *tileA = tiles[0][b], *tileB = tiles[1][b];
 
     if (!real) {
@@ -106,35 +96,12 @@ __global__ void __launch_bounds__(P_NT, (SW * SH <= 1) ? J2P_PROJ_MIN_CTAS : 2) 
     float z[ZH][ZW];
     float v[8], mean[8];
     if constexpr (SW > 0) {
-        unsigned key = 0xffffffffu;
-#pragma unroll
-        for (int sy = 0; sy < SH; sy++) {
-            const size_t gi = (size_t)(cy * SH + sy) * W + (size_t)bx * 8 * SW;
-            const float4 *xr = reinterpret_cast<const float4 *>(P.x + gi);
-            const float4 *pr = reinterpret_cast<const float4 *>(P.xp + gi);
-            const float4 *gr = reinterpret_cast<const float4 *>(P.g + gi);
-#pragma unroll
-            for (int k = 0; k < SW * 2; k++) {
-                float4 a, p, g;
-                if constexpr (SW == 1 && SH == 1) {
-                    a = ra[k]; p = rp[k]; g = rg[k];
-                } else {
-                    a = xr[k]; p = pr[k]; g = gr[k];
-                }
-                z[sy][k * 4 + 0] = stepper.fast(a.x, p.x, g.x, key);
-                z[sy][k * 4 + 1] = stepper.fast(a.y, p.y, g.y, key);
-                z[sy][k * 4 + 2] = stepper.fast(a.z, p.z, g.z, key);
-                z[sy][k * 4 + 3] = stepper.fast(a.w, p.w, g.w, key);
-            }
-        }
-        if (stepper.stepping && !(norm_ok && key >= QDIV_KEY_MIN)) {   // outside the proven range: IEEE division
-#pragma unroll
-            for (int sy = 0; sy < SH; sy++) {
-                const size_t gi = (size_t)(cy * SH + sy) * W + (size_t)bx * 8 * SW;
-#pragma unroll
-                for (int k = 0; k < SW * 8; k++) z[sy][k] = stepper(P.x[gi + k], P.xp[gi + k], P.g[gi + k]);
-            }
-        }
+        step_footprint(stepper, z, [&](int sy, int k) {
+            if constexpr (SW == 1 && SH == 1) return Px4{ra[k], rp[k], rg[k]};
+            const size_t gi = (size_t)(cy * SH + sy) * W + (size_t)bx * 8 * SW + (size_t)k * 4;
+            return Px4{*reinterpret_cast<const float4 *>(P.x + gi), *reinterpret_cast<const float4 *>(P.xp + gi),
+                       *reinterpret_cast<const float4 *>(P.g + gi)};
+        });
 #pragma unroll
         for (int i = 0; i < 8; i++) {
             if (SW * SH > 1 || P.resample) {
@@ -178,44 +145,13 @@ __global__ void __launch_bounds__(P_NT, (SW * SH <= 1) ? J2P_PROJ_MIN_CTAS : 2) 
     fdct8x8_rows(v, tileA, j);
 
     // ---- clamp to the quantisation interval (compute.c:323-331); DCT-distance residual ---------
-    const int dw[4] = {draw.x, draw.y, draw.z, draw.w};
-    float qv[8], qqv[8], rqv[8];
-    {
-        const float4 *t0 = reinterpret_cast<const float4 *>(&sq[0][j * 8]);
-        const float4 *t1 = reinterpret_cast<const float4 *>(&sq[1][j * 8]);
-        const float4 *t2 = reinterpret_cast<const float4 *>(&sq[2][j * 8]);
-#pragma unroll
-        for (int k = 0; k < 2; k++) {
-            const float4 a = t0[k], bq = t1[k], cq = t2[k];
-            qv[k * 4] = a.x; qv[k * 4 + 1] = a.y; qv[k * 4 + 2] = a.z; qv[k * 4 + 3] = a.w;
-            qqv[k * 4] = bq.x; qqv[k * 4 + 1] = bq.y; qqv[k * 4 + 2] = bq.z; qqv[k * 4 + 3] = bq.w;
-            rqv[k * 4] = cq.x; rqv[k * 4 + 1] = cq.y; rqv[k * 4 + 2] = cq.z; rqv[k * 4 + 3] = cq.w;
-        }
-    }
     float r[8], num[8];
-    unsigned rkey = 0xffffffffu;
-#pragma unroll
-    for (int i = 0; i < 8; i++) {
-        const int di = (i & 1) ? (dw[i >> 1] >> 16) : (int)(short)(dw[i >> 1] & 0xffff);
-        const float d = (float)di;
-        const float q = qv[i];
-        const float lo = fmul(fsub(d, 0.5f), q), hi = fmul(fadd(d, 0.5f), q);
-        float t = v[i];
-        t = t > hi ? hi : (t < lo ? lo : t);
-        v[i] = t;
-        num[i] = fsub(t, fmul(d, q));                                        // compute.c:47
-        rkey = min(rkey, qdiv_key(num[i]));
-        r[i] = qdiv_core(num[i], qqv[i], rqv[i]);                            // compute.c:49; q*q in [1, 2^32] is always a valid divisor
-    }
-    if (rkey < QDIV_KEY_MIN) {                                               // a residual below 2^-60: IEEE division
-#pragma unroll
-        for (int i = 0; i < 8; i++) r[i] = fdiv(num[i], qqv[i]);
-    }
+    clamp_residual(v, r, num, draw, &sq[0][0], j);
     if (F.log_on && P.use_prob) {
         // objective term of the NEXT iteration: sum of (residual/q)^2 (compute_simd_step.c:22-26), fp64
         double loc = 0.;
 #pragma unroll
-        for (int i = 0; i < 8; i++) loc = __dadd_rn(loc, (double)fsq(fdiv(num[i], qv[i])));
+        for (int i = 0; i < 8; i++) loc = __dadd_rn(loc, (double)fsq(fdiv(num[i], sq[0][j * 8 + i])));
         const unsigned gmask = 0xffu << (tid & 24);
         loc = __dadd_rn(loc, __shfl_xor_sync(gmask, loc, 1));
         loc = __dadd_rn(loc, __shfl_xor_sync(gmask, loc, 2));
@@ -313,20 +249,63 @@ __global__ void k_init_plane(const float *fdata, float *x, float *xp, int W, int
     }
 }
 
+// Frame pixels of a plane that no coefficient block covers (1080p: luma rows 1080..1087) are only
+// stepped: compute_projection never visits them (compute.c:349-350).  (cwf, chf) = (sw cw, sh ch) is
+// the covered extent; the region is the bottom band (rows >= chf, full width) plus the right band
+// (rows < chf, columns >= cwf).  The tiled kernels leave these pixels to this kernel.
+__global__ void k_step_uncovered(const __grid_constant__ FrameDev F, const int c, const float factor, const int cwf, const int chf) {
+    const PlaneDev &P = F.pl[c];
+    const int W = F.W, H = F.H;
+    const Stepper stepper(factor, F.step, F.norms[c], 0.f);
+    const unsigned bottom = (unsigned)(H - chf) * (unsigned)W, right_w = (unsigned)(W - cwf);
+    const unsigned n = bottom + (unsigned)chf * right_w;
+    for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        unsigned px, py;
+        if (i < bottom) {
+            py = (unsigned)chf + i / (unsigned)W;
+            px = i % (unsigned)W;
+        } else {
+            const unsigned k = i - bottom;
+            py = k / right_w;
+            px = (unsigned)cwf + k % right_w;
+        }
+        const size_t gi = (size_t)py * W + px;
+        P.xp[gi] = stepper(P.x[gi], P.xp[gi], P.g[gi]);
+    }
+}
+
 // ------------------------------------------------------------------------------------------
 // host-side launchers
 // ------------------------------------------------------------------------------------------
-// 2x2 planes (4:2:0 chroma) go through kernels_project_tile22.cu (coalesced staging; round 2:
-// bit-identical on the whole GPU suite, 8K 4:2:0 projection 508 -> 362 us, profiles/r02_notes.md).
-// J2P_PROJ_TILE22=0 selects the register-footprint kernel k_project<2,2> instead (A/B aid; it is
-// also what the objective-logging build uses).
-static bool g_tile22 = true;
-
 cudaError_t configure_project_kernels() {
-    const char *e = getenv("J2P_PROJ_TILE22");
-    g_tile22 = !(e && *e == '0');
     const cudaError_t rc = configure_project_tma();
     return rc != cudaSuccess ? rc : configure_project_tile22();
+}
+
+// The one place that decides which kernel projects plane c.  Objective logging needs the
+// k_project<SW, SH> build that also sums the log terms; otherwise 1x1 planes go through the
+// cp.async tile kernel (or, with J2P_PROJ_TMA=1 and tensor maps, the TMA kernel), 2x2 planes
+// (4:2:0 chroma) through the tile22 kernel and every other sampling through k_project<SW, SH>.
+enum class ProjKernel { tile, tile22, tma, generic };
+
+static ProjKernel project_kernel(const FrameDev &F, int c) {
+    const PlaneDev &P = F.pl[c];
+    if (F.log_on) return ProjKernel::generic;
+    if (P.sw == 1 && P.sh == 1) return F.host_maps != nullptr && project_tma_enabled() ? ProjKernel::tma : ProjKernel::tile;
+    if (P.sw == 2 && P.sh == 2) return ProjKernel::tile22;
+    return ProjKernel::generic;
+}
+
+// Units of work of plane c's projection kernel per block row, each of which delivers its share of
+// the strip border rows to the neighbours (strip_border_done); 0: the kernel does not deliver them.
+int project_border_units(const FrameDev &F, int c) {
+    const int bw = F.pl[c].cw >> 3;
+    switch (project_kernel(F, c)) {
+        case ProjKernel::tile: return (bw + PT_NB - 1) / PT_NB;
+        case ProjKernel::tile22: return (bw + P22_NB - 1) / P22_NB;
+        case ProjKernel::tma: return (bw + TP_NB - 1) / TP_NB;
+        default: return 0;
+    }
 }
 
 // strip sessions: fold the per-rank sums of g^2 in rank order (deterministic), then the norms of
@@ -346,6 +325,27 @@ cudaError_t launch_fold_sums(const double *sums_by_rank, int nranks, int nc, flo
     return cudaGetLastError();
 }
 
+static cudaError_t launch_project_generic(const FrameDev &F, int c, float factor, cudaStream_t s) {
+    const PlaneDev &P = F.pl[c];
+    const int tw = 8 * P_BW * P.sw, th = 8 * P_BH * P.sh;
+    const dim3 grid((F.W + tw - 1) / tw, (F.H + th - 1) / th);
+    const ProjPlane G = {c, (int)grid.x};
+    if (P.sw == 1 && P.sh == 1) k_project<1, 1><<<grid, P_NT, 0, s>>>(F, G, factor);
+    else if (P.sw == 2 && P.sh == 2) k_project<2, 2><<<grid, P_NT, 0, s>>>(F, G, factor);
+    else if (P.sw == 2 && P.sh == 1) k_project<2, 1><<<grid, P_NT, 0, s>>>(F, G, factor);
+    else if (P.sw == 1 && P.sh == 2) k_project<1, 2><<<grid, P_NT, 0, s>>>(F, G, factor);
+    else k_project<0, 0><<<grid, P_NT, 0, s>>>(F, G, factor);
+    return cudaGetLastError();
+}
+
+static cudaError_t launch_step_uncovered(const FrameDev &F, int c, float factor, int cwf, int chf, cudaStream_t s) {
+    const size_t n = (size_t)(F.H - chf) * F.W + (size_t)chf * (F.W - cwf);
+    int blocks = (int)((n + 255) / 256);
+    if (blocks > 148 * 8) blocks = 148 * 8;
+    k_step_uncovered<<<blocks, 256, 0, s>>>(F, c, factor, cwf, chf);
+    return cudaGetLastError();
+}
+
 // *nlaunch: number of kernels launched (planes of one geometry share a launch)
 cudaError_t launch_project(const FrameDev &Fin, float factor, cudaStream_t s, int *nlaunch) {
     *nlaunch = 0;
@@ -360,48 +360,31 @@ cudaError_t launch_project(const FrameDev &Fin, float factor, cudaStream_t s, in
         }
         F.H = F.t1 - F.t0;
     }
-    for (int c = 0; c < F.nc; c++) {
+    for (int c = 0, count; c < F.nc; c += count) {
         const PlaneDev &P = F.pl[c];
-        const int tw = 8 * P_BW * P.sw, th = 8 * P_BH * P.sh;
-        ProjPlane G;
-        G.c = c;
-        G.gx = (F.W + tw - 1) / tw;
-        const dim3 grid(G.gx, (F.H + th - 1) / th);
-        const int before = *nlaunch;
-        if (F.log_on && P.sw == 1 && P.sh == 1) {
-            k_project<1, 1><<<grid, P_NT, 0, s>>>(F, G, factor);                // the variant that also sums the log terms
-        } else if (P.sw == 1 && P.sh == 1) {
-            int count = 1;      // following planes of identical geometry ride in the same launch (grid.z)
-            while (c + count < F.nc && F.pl[c + count].sw == 1 && F.pl[c + count].sh == 1 && F.pl[c + count].cw == P.cw &&
-                   F.pl[c + count].ch == P.ch)
-                count++;
-            // persistent TMA-fed kernel where the session has tensor maps; it takes the unrestricted frame
-            const bool tma = Fin.host_maps != nullptr && project_tma_enabled();
-            if (tma) {
-                const cudaError_t et = launch_project_tma(Fin, *static_cast<const TileMaps *>(Fin.host_maps), c, count, Fin.buf_sel, factor, s);
-                if (et != cudaSuccess) return et;
+        const ProjKernel k = project_kernel(F, c);
+        count = 1;              // following planes of identical geometry ride in the same tiled launch (grid.z)
+        while (k != ProjKernel::generic && c + count < F.nc && project_kernel(F, c + count) == k && F.pl[c + count].cw == P.cw &&
+               F.pl[c + count].ch == P.ch)
+            count++;
+        cudaError_t e = cudaSuccess;
+        switch (k) {
+            // the TMA kernel takes the unrestricted frame: it adds F.t0 itself
+            case ProjKernel::tma: e = launch_project_tma(Fin, *static_cast<const TileMaps *>(Fin.host_maps), c, count, Fin.buf_sel, factor, s); break;
+            case ProjKernel::tile: e = launch_project_tile(F, c, count, factor, s); break;
+            case ProjKernel::tile22: e = launch_project_tile22(F, c, count, factor, s); break;
+            case ProjKernel::generic: e = launch_project_generic(F, c, factor, s); break;
+        }
+        if (e != cudaSuccess) return e;
+        *nlaunch += 1;
+        if (k == ProjKernel::generic) continue;         // k_project<> steps the uncovered pixels itself
+        for (int q = c; q < c + count; q++) {
+            const int cwf = F.pl[q].sw * F.pl[q].cw, chf = F.pl[q].sh * F.pl[q].ch;
+            if (cwf < F.W || chf < F.H) {
+                if ((e = launch_step_uncovered(F, q, factor, cwf, chf, s)) != cudaSuccess) return e;
                 *nlaunch += 1;
             }
-            const cudaError_t eb = launch_project_tile(F, c, count, factor, s, nlaunch, tma);
-            if (eb != cudaSuccess) return eb;
-            c += count - 1;
         }
-        else if (P.sw == 2 && P.sh == 2 && g_tile22 && !F.log_on) {
-            int count = 1;      // Cb and Cr share one launch
-            while (c + count < F.nc && F.pl[c + count].sw == 2 && F.pl[c + count].sh == 2 && F.pl[c + count].cw == P.cw &&
-                   F.pl[c + count].ch == P.ch)
-                count++;
-            const cudaError_t eb = launch_project_tile22(F, c, count, factor, s, nlaunch);
-            if (eb != cudaSuccess) return eb;
-            c += count - 1;
-        }
-        else if (P.sw == 2 && P.sh == 2) k_project<2, 2><<<grid, P_NT, 0, s>>>(F, G, factor);
-        else if (P.sw == 2 && P.sh == 1) k_project<2, 1><<<grid, P_NT, 0, s>>>(F, G, factor);
-        else if (P.sw == 1 && P.sh == 2) k_project<1, 2><<<grid, P_NT, 0, s>>>(F, G, factor);
-        else k_project<0, 0><<<grid, P_NT, 0, s>>>(F, G, factor);
-        if (*nlaunch == before) *nlaunch += 1;                       // one of the direct k_project<> launches above
-        const cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) return e;
     }
     return cudaSuccess;
 }

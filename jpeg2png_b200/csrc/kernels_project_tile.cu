@@ -23,12 +23,6 @@
 
 namespace j2p {
 
-#ifndef J2P_TILE_BLOCKS
-#define J2P_TILE_BLOCKS 16            // coefficient blocks per CTA tile (16 or 32: the tables and the norm take 96 threads).  Measured at 4K
-                                      // (profiles/r02_ab_gradient_geometry.txt): 16-block tiles in eight 4-warp CTAs per SM 130.1 us, 32-block tiles in
-                                      // four 8-warp CTAs 133.0 us — same resident warps, half as many warps behind each of the two CTA barriers
-#endif
-constexpr int PT_NB = J2P_TILE_BLOCKS;
 constexpr int PT_NT = PT_NB * 8;      // 8 threads per block
 constexpr int PT_C4 = PT_NB * 2;      // float4 columns per tile row
 constexpr int PT_SH = PT_NB == 32 ? 6 : (PT_NB == 16 ? 5 : 7);   // log2(PT_C4)
@@ -82,22 +76,11 @@ __global__ void __launch_bounds__(PT_NT, J2P_TILE_MIN_CTAS) k_project_tile(const
     const bool real = b < nbx;
     int4 draw = make_int4(0, 0, 0, 0);
     if (real) draw = __ldg(reinterpret_cast<const int4 *>(P.data + ((size_t)(by * bw + bx0 + b) * 64 + j * 8)));   // 512 B per warp, coalesced
-    if (tid < 64) {
-        sq[0][tid] = F.q[c][tid];
-        sq[1][tid] = F.qq[c][tid];
-        sq[2][tid] = F.rqq[c][tid];
-    }
-    if (tid >= 64 && tid < 96) strip_norm(F, c, snorm, tid - 64);    // whole frame: what k_gradient left; strips: fold of every rank's sums
+    stage_tables(F, c, &sq[0][0], snorm, tid);
     cp_async_wait<0>();
     __syncthreads();
 
-    Stepper stepper;
-    stepper.factor = factor;
-    stepper.step = F.step;
-    stepper.norm = snorm[0];
-    stepper.rn = snorm[1];
-    stepper.stepping = stepper.norm != 0.f;                        // compute.c:211
-    const bool norm_ok = qdiv_divisor_ok(stepper.norm);
+    const Stepper stepper(factor, F.step, snorm[0], snorm[1]);
     const bool use_prob = P.use_prob != 0;
     constexpr bool resample = RES;
     const unsigned gmask = 0xffu << (tid & 24);
@@ -105,78 +88,28 @@ __global__ void __launch_bounds__(PT_NT, J2P_TILE_MIN_CTAS) k_project_tile(const
 
     if (real) {
         // ---- stepped point (compute.c:436, :213) from this thread's row of the tile --------------
-        float z[8], v[8], mean[8];
-        {
-            unsigned key = 0xffffffffu;
-#pragma unroll
-            for (int h = 0; h < 2; h++) {
-                const int pc = (2 * b + h) ^ j;
-                const float4 a = sx[j][pc], p = sp[j][pc], g = sg[j][pc];
-                z[h * 4 + 0] = stepper.fast(a.x, p.x, g.x, key);
-                z[h * 4 + 1] = stepper.fast(a.y, p.y, g.y, key);
-                z[h * 4 + 2] = stepper.fast(a.z, p.z, g.z, key);
-                z[h * 4 + 3] = stepper.fast(a.w, p.w, g.w, key);
-            }
-            if (stepper.stepping && !(norm_ok && key >= QDIV_KEY_MIN)) {   // outside the proven range: IEEE division
-#pragma unroll
-                for (int h = 0; h < 2; h++) {
-                    const int pc = (2 * b + h) ^ j;
-                    const float4 a = sx[j][pc], p = sp[j][pc], g = sg[j][pc];
-                    z[h * 4 + 0] = stepper(a.x, p.x, g.x);
-                    z[h * 4 + 1] = stepper(a.y, p.y, g.y);
-                    z[h * 4 + 2] = stepper(a.z, p.z, g.z);
-                    z[h * 4 + 3] = stepper(a.w, p.w, g.w);
-                }
-            }
-        }
+        float z[1][8], v[8], mean[8];
+        step_footprint(stepper, z, [&](int, int h) {
+            const int pc = (2 * b + h) ^ j;
+            return Px4{sx[j][pc], sp[j][pc], sg[j][pc]};
+        });
 #pragma unroll
         for (int i = 0; i < 8; i++) {
             if (resample) {                                        // sampling 1x1 on a coefficient grid smaller than the frame
-                const float m = fadd(0.f, z[i]);                   // compute.c:351-359 with one sample: (0 + z) / 1
+                const float m = fadd(0.f, z[0][i]);                // compute.c:351-359 with one sample: (0 + z) / 1
                 mean[i] = m;
                 v[i] = m;
             } else {
                 mean[i] = 0.f;
-                v[i] = z[i];
+                v[i] = z[0][i];
             }
         }
 
         fdct8x8_rows(v, tile, j, gmask);
 
         // ---- clamp to the quantisation interval (compute.c:323-331); residual (compute.c:47-49) --
-        const int dw[4] = {draw.x, draw.y, draw.z, draw.w};
         float r[8], num[8];
-        unsigned rkey = 0xffffffffu;
-        {
-            const float4 *t0 = reinterpret_cast<const float4 *>(&sq[0][j * 8]);
-            const float4 *t1 = reinterpret_cast<const float4 *>(&sq[1][j * 8]);
-            const float4 *t2 = reinterpret_cast<const float4 *>(&sq[2][j * 8]);
-            float qv[8], qqv[8], rqv[8];
-#pragma unroll
-            for (int k = 0; k < 2; k++) {
-                const float4 a = t0[k], bq = t1[k], cq = t2[k];
-                qv[k * 4] = a.x; qv[k * 4 + 1] = a.y; qv[k * 4 + 2] = a.z; qv[k * 4 + 3] = a.w;
-                qqv[k * 4] = bq.x; qqv[k * 4 + 1] = bq.y; qqv[k * 4 + 2] = bq.z; qqv[k * 4 + 3] = bq.w;
-                rqv[k * 4] = cq.x; rqv[k * 4 + 1] = cq.y; rqv[k * 4 + 2] = cq.z; rqv[k * 4 + 3] = cq.w;
-            }
-#pragma unroll
-            for (int i = 0; i < 8; i++) {
-                const int di = (i & 1) ? (dw[i >> 1] >> 16) : (int)(short)(dw[i >> 1] & 0xffff);
-                const float d = (float)di;
-                const float q = qv[i];
-                const float lo = fmul(fsub(d, 0.5f), q), hi = fmul(fadd(d, 0.5f), q);
-                float t = v[i];
-                t = t > hi ? hi : (t < lo ? lo : t);
-                v[i] = t;
-                num[i] = fsub(t, fmul(d, q));
-                rkey = min(rkey, qdiv_key(num[i]));
-                r[i] = qdiv_core(num[i], qqv[i], rqv[i]);
-            }
-            if (rkey < QDIV_KEY_MIN) {                             // a residual below 2^-60: IEEE division
-#pragma unroll
-                for (int i = 0; i < 8; i++) r[i] = fdiv(num[i], qqv[i]);
-            }
-        }
+        clamp_residual(v, r, num, draw, &sq[0][0], j);
 
         idct8x8_rows(v, tile, j, gmask);
         if (use_prob) idct8x8_rows(r, tile, j, gmask);
@@ -184,7 +117,7 @@ __global__ void __launch_bounds__(PT_NT, J2P_TILE_MIN_CTAS) k_project_tile(const
         // ---- results into this thread's own cells of the staging tiles ---------------------------
         if (resample) {
 #pragma unroll
-            for (int i = 0; i < 8; i++) v[i] = fadd(fsub(z[i], mean[i]), v[i]);   // compute.c:390-403
+            for (int i = 0; i < 8; i++) v[i] = fadd(fsub(z[0][i], mean[i]), v[i]);   // compute.c:390-403
         }
         const float pa = P.p_alpha;
 #pragma unroll
@@ -208,84 +141,16 @@ __global__ void __launch_bounds__(PT_NT, J2P_TILE_MIN_CTAS) k_project_tile(const
         }
     }
 
-    // ---- strips over peer memory: the strip's first / last two rows also go straight into the
-    // neighbours' halo rows (NVLink stores), and the last border CTA of the iteration raises their flag
-    const StripSync &S = F.sync;
-    if (S.nranks > 1 && S.fused_halo) {
-        const bool top = by == 0 && S.has_up, bottom = by == (int)gridDim.y - 1 && S.has_down;
-        if (top || bottom) {
-            for (int e = tid; e < 4 * PT_C4; e += PT_NT) {                // 2 rows x 64 pieces, top then bottom
-                const int side = e >> (PT_SH + 1), r = (e >> PT_SH) & 1, c4 = e & (PT_C4 - 1);
-                if (c4 >= valid_c4 || !(side ? bottom : top)) continue;
-                const int row = side ? 6 + r : r;
-                float *dst = (side ? S.down_dst[c] : S.up_dst[c]) + (size_t)r * W + (size_t)bx0 * 8 + (size_t)c4 * 4;
-                *reinterpret_cast<float4 *>(dst) = sx[row][c4 ^ row];
-            }
-            if (top) strip_border_done(S, 0);
-            if (bottom) strip_border_done(S, 1);
-        }
-    }
+    // ---- strips over peer memory: the tile's border rows into the neighbours' halo rows -----------
+    deliver_border_rows<PT_NT, 8, PT_C4>(F, c, by, W, valid_c4, bx0, [&](int row, int c4) { return sx[row][c4 ^ row]; });
 }
-
-// Frame pixels of a 1x1 plane that no coefficient block covers (1080p: luma rows 1080..1087) are
-// only stepped: compute_projection never visits them (compute.c:349-350).  The region is the
-// bottom band (rows >= ch, full width) plus the right band (rows < ch, columns >= cw).
-__global__ void k_step_uncovered(const __grid_constant__ FrameDev F, const int c, const float factor) {
-    const PlaneDev &P = F.pl[c];
-    const int W = F.W, H = F.H;
-    Stepper stepper;
-    stepper.factor = factor;
-    stepper.step = F.step;
-    stepper.norm = F.norms[c];
-    stepper.rn = 0.f;
-    stepper.stepping = stepper.norm != 0.f;
-    const unsigned bottom = (unsigned)(H - P.ch) * (unsigned)W, right_w = (unsigned)(W - P.cw);
-    const unsigned n = bottom + (unsigned)P.ch * right_w;
-    for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-        unsigned px, py;
-        if (i < bottom) {
-            py = (unsigned)P.ch + i / (unsigned)W;
-            px = i % (unsigned)W;
-        } else {
-            const unsigned k = i - bottom;
-            py = k / right_w;
-            px = (unsigned)P.cw + k % right_w;
-        }
-        const size_t gi = (size_t)py * W + px;
-        P.xp[gi] = stepper(P.x[gi], P.xp[gi], P.g[gi]);
-    }
-}
-
-static cudaError_t launch_step_uncovered(const FrameDev &F, int c, float factor, cudaStream_t s) {
-    const PlaneDev &P = F.pl[c];
-    const size_t n = (size_t)(F.H - P.ch) * F.W + (size_t)P.ch * (F.W - P.cw);
-    int blocks = (int)((n + 255) / 256);
-    if (blocks > 148 * 8) blocks = 148 * 8;
-    k_step_uncovered<<<blocks, 256, 0, s>>>(F, c, factor);
-    return cudaGetLastError();
-}
-
-// CTAs of plane P per block row: what calls strip_border_done per side and iteration (session.cu counts them)
-int project_tile_border_units(const PlaneDev &P) { return ((P.cw >> 3) + PT_NB - 1) / PT_NB; }
 
 // F: already restricted to the rows the session owns (launch_project).  Projects planes
 // c .. c+count-1, which must all be 1x1 planes with the same coefficient grid.
-// uncovered_only: the tiles have been projected by the TMA kernel; only the stepped-only pixels remain
-cudaError_t launch_project_tile(const FrameDev &F, int c, int count, float factor, cudaStream_t s, int *nlaunch, bool uncovered_only) {
+cudaError_t launch_project_tile(const FrameDev &F, int c, int count, float factor, cudaStream_t s) {
     const PlaneDev &P = F.pl[c];
-    const int bw = P.cw >> 3, bh = P.ch >> 3;
-    const dim3 grid((bw + PT_NB - 1) / PT_NB, bh, count);
-    cudaError_t e = cudaSuccess;
-    if (!uncovered_only) {
-        e = P.resample ? launch_chain(k_project_tile<true>, grid, dim3(PT_NT), 0, s, F, c, factor) : launch_chain(k_project_tile<false>, grid, dim3(PT_NT), 0, s, F, c, factor);
-        *nlaunch += 1;
-    }
-    for (int k = c; k < c + count && e == cudaSuccess; k++)
-        if (F.pl[k].cw < F.W || F.pl[k].ch < F.H) {
-            e = launch_step_uncovered(F, k, factor, s);
-            *nlaunch += 1;
-        }
-    return e;
+    const dim3 grid(((P.cw >> 3) + PT_NB - 1) / PT_NB, P.ch >> 3, count);
+    return P.resample ? launch_chain(k_project_tile<true>, grid, dim3(PT_NT), 0, s, F, c, factor) : launch_chain(k_project_tile<false>, grid, dim3(PT_NT), 0, s, F, c, factor);
 }
 
 }  // namespace j2p

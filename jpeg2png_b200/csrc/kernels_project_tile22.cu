@@ -24,7 +24,6 @@
 
 namespace j2p {
 
-constexpr int P22_NB = 16;                 // coefficient blocks per CTA tile (16 x 1)
 constexpr int P22_NT = P22_NB * 8;         // 128 threads
 constexpr int P22_C4 = P22_NB * 4;         // float4 columns per frame row of the tile (256 pixels)
 constexpr int P22_G4 = P22_NB * 2;         // float4 columns per coefficient row of the tile (128 samples)
@@ -79,22 +78,11 @@ __global__ void __launch_bounds__(P22_NT, 3) k_project_tile22(const __grid_const
     const bool real = b < nbx;
     int4 draw = make_int4(0, 0, 0, 0);
     if (real) draw = __ldg(reinterpret_cast<const int4 *>(P.data + ((size_t)(by * bw + bx0 + b) * 64 + j * 8)));
-    if (tid < 64) {
-        sq[tid] = F.q[c][tid];
-        sq[64 + tid] = F.qq[c][tid];
-        sq[128 + tid] = F.rqq[c][tid];
-    }
-    if (tid >= 64 && tid < 96) strip_norm(F, c, snorm, tid - 64);    // whole frame: what k_gradient left; strips: fold of every rank's sums
+    stage_tables(F, c, sq, snorm, tid);
     cp_async_wait<0>();
     __syncthreads();
 
-    Stepper stepper;
-    stepper.factor = factor;
-    stepper.step = F.step;
-    stepper.norm = snorm[0];
-    stepper.rn = snorm[1];
-    stepper.stepping = stepper.norm != 0.f;                          // compute.c:211
-    const bool norm_ok = qdiv_divisor_ok(stepper.norm);
+    const Stepper stepper(factor, F.step, snorm[0], snorm[1]);
     const bool use_prob = P.use_prob != 0;
     const unsigned gmask = 0xffu << (tid & 24);
     float *tile = tiles + b * TILE_STRIDE;
@@ -102,37 +90,10 @@ __global__ void __launch_bounds__(P22_NT, 3) k_project_tile22(const __grid_const
     if (real) {
         // ---- stepped point of the 2 x 16 footprint (compute.c:436, :213) --------------------------
         float z[2][16], v[8], mean[8];
-        {
-            unsigned key = 0xffffffffu;
-#pragma unroll
-            for (int sy = 0; sy < 2; sy++) {
-                const int rowbase = (2 * j + sy) * P22_C4;
-#pragma unroll
-                for (int k = 0; k < 4; k++) {
-                    const int pc = rowbase + ((4 * b + k) ^ j);      // (row >> 1) & 7 == j
-                    const float4 a = sx[pc], p = sp[pc], g = sg[pc];
-                    z[sy][k * 4 + 0] = stepper.fast(a.x, p.x, g.x, key);
-                    z[sy][k * 4 + 1] = stepper.fast(a.y, p.y, g.y, key);
-                    z[sy][k * 4 + 2] = stepper.fast(a.z, p.z, g.z, key);
-                    z[sy][k * 4 + 3] = stepper.fast(a.w, p.w, g.w, key);
-                }
-            }
-            if (stepper.stepping && !(norm_ok && key >= QDIV_KEY_MIN)) {   // outside the proven range: IEEE division
-#pragma unroll
-                for (int sy = 0; sy < 2; sy++) {
-                    const int rowbase = (2 * j + sy) * P22_C4;
-#pragma unroll
-                    for (int k = 0; k < 4; k++) {
-                        const int pc = rowbase + ((4 * b + k) ^ j);
-                        const float4 a = sx[pc], p = sp[pc], g = sg[pc];
-                        z[sy][k * 4 + 0] = stepper(a.x, p.x, g.x);
-                        z[sy][k * 4 + 1] = stepper(a.y, p.y, g.y);
-                        z[sy][k * 4 + 2] = stepper(a.z, p.z, g.z);
-                        z[sy][k * 4 + 3] = stepper(a.w, p.w, g.w);
-                    }
-                }
-            }
-        }
+        step_footprint(stepper, z, [&](int sy, int k) {
+            const int pc = (2 * j + sy) * P22_C4 + ((4 * b + k) ^ j);   // (row >> 1) & 7 == j
+            return Px4{sx[pc], sp[pc], sg[pc]};
+        });
         // block-row means over the 2 x 2 samples, sy outer, sx inner (compute.c:351-360)
 #pragma unroll
         for (int i = 0; i < 8; i++) {
@@ -149,39 +110,8 @@ __global__ void __launch_bounds__(P22_NT, 3) k_project_tile22(const __grid_const
         fdct8x8_rows(v, tile, j, gmask);
 
         // ---- clamp to the quantisation interval (compute.c:323-331); residual (compute.c:47-49) --
-        const int dw[4] = {draw.x, draw.y, draw.z, draw.w};
         float r[8], num[8];
-        unsigned rkey = 0xffffffffu;
-        {
-            const float4 *t0 = reinterpret_cast<const float4 *>(&sq[j * 8]);
-            const float4 *t1 = reinterpret_cast<const float4 *>(&sq[64 + j * 8]);
-            const float4 *t2 = reinterpret_cast<const float4 *>(&sq[128 + j * 8]);
-            float qv[8], qqv[8], rqv[8];
-#pragma unroll
-            for (int k = 0; k < 2; k++) {
-                const float4 a = t0[k], bq = t1[k], cq = t2[k];
-                qv[k * 4] = a.x; qv[k * 4 + 1] = a.y; qv[k * 4 + 2] = a.z; qv[k * 4 + 3] = a.w;
-                qqv[k * 4] = bq.x; qqv[k * 4 + 1] = bq.y; qqv[k * 4 + 2] = bq.z; qqv[k * 4 + 3] = bq.w;
-                rqv[k * 4] = cq.x; rqv[k * 4 + 1] = cq.y; rqv[k * 4 + 2] = cq.z; rqv[k * 4 + 3] = cq.w;
-            }
-#pragma unroll
-            for (int i = 0; i < 8; i++) {
-                const int di = (i & 1) ? (dw[i >> 1] >> 16) : (int)(short)(dw[i >> 1] & 0xffff);
-                const float d = (float)di;
-                const float q = qv[i];
-                const float lo = fmul(fsub(d, 0.5f), q), hi = fmul(fadd(d, 0.5f), q);
-                float t = v[i];
-                t = t > hi ? hi : (t < lo ? lo : t);
-                v[i] = t;
-                num[i] = fsub(t, fmul(d, q));
-                rkey = min(rkey, qdiv_key(num[i]));
-                r[i] = qdiv_core(num[i], qqv[i], rqv[i]);
-            }
-            if (rkey < QDIV_KEY_MIN) {                               // a residual below 2^-60: IEEE division
-#pragma unroll
-                for (int i = 0; i < 8; i++) r[i] = fdiv(num[i], qqv[i]);
-            }
-        }
+        clamp_residual(v, r, num, draw, sq, j);
 
         idct8x8_rows(v, tile, j, gmask);
         if (use_prob) idct8x8_rows(r, tile, j, gmask);
@@ -227,49 +157,8 @@ __global__ void __launch_bounds__(P22_NT, 3) k_project_tile22(const __grid_const
         }
     }
 
-    // ---- strips over peer memory: border rows into the neighbours' halo rows (kernels_project_tile.cu)
-    const StripSync &S = F.sync;
-    if (S.nranks > 1 && S.fused_halo) {
-        const bool top = by == 0 && S.has_up, bottom = by == (int)gridDim.y - 1 && S.has_down;
-        if (top || bottom) {
-            for (int e = tid; e < 4 * P22_C4; e += P22_NT) {             // 2 rows x 64 pieces, top then bottom
-                const int side = e / (2 * P22_C4), r = (e / P22_C4) & 1, c4 = e % P22_C4;
-                if (c4 >= valid_c4 || !(side ? bottom : top)) continue;
-                const int row = side ? 14 + r : r;
-                float *dst = (side ? S.down_dst[c] : S.up_dst[c]) + (size_t)r * W + (size_t)bx0 * 16 + (size_t)c4 * 4;
-                *reinterpret_cast<float4 *>(dst) = sx[row * P22_C4 + (c4 ^ ((row >> 1) & 7))];
-            }
-            if (top) strip_border_done(S, 0);
-            if (bottom) strip_border_done(S, 1);
-        }
-    }
-}
-
-// frame pixels of a 2x2 plane beyond its coefficient grid (W > 2 cw or H > 2 ch): step only
-__global__ void k_step_uncovered22(const __grid_constant__ FrameDev F, const int c, const float factor) {
-    const PlaneDev &P = F.pl[c];
-    const int W = F.W, H = F.H, cwf = 2 * P.cw, chf = 2 * P.ch;
-    Stepper stepper;
-    stepper.factor = factor;
-    stepper.step = F.step;
-    stepper.norm = F.norms[c];
-    stepper.rn = 0.f;
-    stepper.stepping = stepper.norm != 0.f;
-    const unsigned bottom = (unsigned)(H - chf) * (unsigned)W, right_w = (unsigned)(W - cwf);
-    const unsigned n = bottom + (unsigned)chf * right_w;
-    for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-        unsigned px, py;
-        if (i < bottom) {
-            py = (unsigned)chf + i / (unsigned)W;
-            px = i % (unsigned)W;
-        } else {
-            const unsigned k = i - bottom;
-            py = k / right_w;
-            px = (unsigned)cwf + k % right_w;
-        }
-        const size_t gi = (size_t)py * W + px;
-        P.xp[gi] = stepper(P.x[gi], P.xp[gi], P.g[gi]);
-    }
+    // ---- strips over peer memory: the tile's border rows into the neighbours' halo rows -----------
+    deliver_border_rows<P22_NT, 16, P22_C4>(F, c, by, W, valid_c4, bx0, [&](int row, int c4) { return sx[row * P22_C4 + (c4 ^ ((row >> 1) & 7))]; });
 }
 
 cudaError_t configure_project_tile22() {
@@ -278,24 +167,10 @@ cudaError_t configure_project_tile22() {
 
 // F: already restricted to the rows the session owns (launch_project).  Projects planes
 // c .. c+count-1, which must all be 2x2 planes with the same coefficient grid.
-cudaError_t launch_project_tile22(const FrameDev &F, int c, int count, float factor, cudaStream_t s, int *nlaunch) {
+cudaError_t launch_project_tile22(const FrameDev &F, int c, int count, float factor, cudaStream_t s) {
     const PlaneDev &P = F.pl[c];
-    const int bw = P.cw >> 3, bh = P.ch >> 3;
-    const dim3 grid((bw + P22_NB - 1) / P22_NB, bh, count);
-    cudaError_t e = launch_chain(k_project_tile22, grid, dim3(P22_NT), P22_SMEM, s, F, c, factor);
-    *nlaunch += 1;
-    for (int k = c; k < c + count && e == cudaSuccess; k++) {
-        const PlaneDev &Q = F.pl[k];
-        if (2 * Q.cw < F.W || 2 * Q.ch < F.H) {
-            const size_t n = (size_t)(F.H - 2 * Q.ch) * F.W + (size_t)2 * Q.ch * (F.W - 2 * Q.cw);
-            int blocks = (int)((n + 255) / 256);
-            if (blocks > 148 * 8) blocks = 148 * 8;
-            k_step_uncovered22<<<blocks, 256, 0, s>>>(F, k, factor);
-            e = cudaGetLastError();
-            *nlaunch += 1;
-        }
-    }
-    return e;
+    const dim3 grid(((P.cw >> 3) + P22_NB - 1) / P22_NB, P.ch >> 3, count);
+    return launch_chain(k_project_tile22, grid, dim3(P22_NT), P22_SMEM, s, F, c, factor);
 }
 
 }  // namespace j2p

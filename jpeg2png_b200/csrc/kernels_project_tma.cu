@@ -203,13 +203,7 @@ __global__ void __launch_bounds__(TP_NT, TP_CTAS) k_project_tma(const __grid_con
         const int nbx = min(4, bw - q.bx0);
         const bool real = b < nbx;
         const bool use_prob = info.use_prob != 0;
-        Stepper stepper;
-        stepper.factor = factor;
-        stepper.step = F.step;
-        stepper.norm = snorm[2 * q.z];
-        stepper.rn = snorm[2 * q.z + 1];
-        stepper.stepping = stepper.norm != 0.f;                        // compute.c:211
-        const bool norm_ok = qdiv_divisor_ok(stepper.norm);
+        const Stepper stepper(factor, F.step, snorm[2 * q.z], snorm[2 * q.z + 1]);
         Stepper2 stepper2;
         stepper2.init(stepper, F.one);
         // the tile's quantised coefficients: 16 bytes per thread, 512 contiguous bytes per warp
@@ -229,7 +223,7 @@ __global__ void __launch_bounds__(TP_NT, TP_CTAS) k_project_tma(const __grid_con
                 const f2 y23 = stepper2.fast(pk(a.z, a.w), pk(p.z, p.w), pk(g.z, g.w), key);
                 z[h * 4 + 0] = lo(y01); z[h * 4 + 1] = hi(y01); z[h * 4 + 2] = lo(y23); z[h * 4 + 3] = hi(y23);
             }
-            if (stepper.stepping && !(norm_ok && key >= QDIV_KEY_MIN)) {   // outside the proven range: IEEE division
+            if (stepper.stepping && !(stepper.norm_ok && key >= QDIV_KEY_MIN)) {   // outside the proven range: IEEE division
 #pragma unroll
                 for (int h = 0; h < 2; h++) {
                     const int ci = h ? ci1 : ci0;
@@ -392,18 +386,16 @@ cudaError_t configure_project_tma() {
 
 bool project_tma_enabled() { return g_tma_on; }
 
-// how many units of plane P call strip_border_done per side and iteration (session.cu counts them)
-int project_tma_border_units(const PlaneDev &P) { return ((P.cw >> 3) + 3) / 4; }
-
 // F: the session's frame (NOT restricted to the owned rows: the kernel adds F.t0 itself).  Projects
 // planes c .. c+count-1, which must all be 1x1 planes with the same coefficient grid and have maps.
 cudaError_t launch_project_tma(const FrameDev &F, const TileMaps &M, int c, int count, int xsel, float factor, cudaStream_t s) {
     const PlaneDev &P = F.pl[c];
     const int bw = P.cw >> 3, bh = P.ch >> 3;
-    const int ntiles = ((bw + 3) / 4) * bh * count;                    // warp tiles
+    const int tw = (bw + TP_NB - 1) / TP_NB;                           // warp tiles per block row
+    const int ntiles = tw * bh * count;
     const int ctas = (ntiles + TP_WARPS - 1) / TP_WARPS;
     const int grid = ctas < g_tma_slots ? ctas : g_tma_slots;
-    const unsigned long long mg = 0x100000000ull / (unsigned long long)((bw + 3) / 4);
+    const unsigned long long mg = 0x100000000ull / (unsigned long long)tw;
     const unsigned tw_magic = mg > 0xffffffffull ? 0xffffffffu : (unsigned)mg;                     // one tile per row: t - 1, repaired by the fix-up
     if (P.resample) k_project_tma<true><<<grid, TP_NT, TP_SMEM, s>>>(F, M, c, count, xsel, factor, tw_magic);
     else k_project_tma<false><<<grid, TP_NT, TP_SMEM, s>>>(F, M, c, count, xsel, factor, tw_magic);

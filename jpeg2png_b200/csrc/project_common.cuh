@@ -1,16 +1,35 @@
-// project_common.cuh — pieces shared by the step+projection kernels.
+// project_common.cuh — the block core shared by the step+projection kernels: the stepper, the
+// prologue, the stepped point of a footprint, the clamp with its residual, the 8x8 transforms and
+// the fused-halo delivery of the border rows.  Every projection kernel that has one of these
+// stages uses the function here, so a parity fix is made once.
 #pragma once
 #include <cuda_runtime.h>
 
+#include "kernels.cuh"
 #include "numerics.cuh"
+#include "strip_sync.cuh"
 
 namespace j2p {
+
+// Coefficient blocks in one block row of a tiled projection kernel's unit of work.  Each unit that
+// holds a strip border row delivers its share of it to the neighbour (project_border_units).
+#ifndef J2P_TILE_BLOCKS
+#define J2P_TILE_BLOCKS 16            // k_project_tile (16 or 32: the tables and the norm take 96 threads).  Measured at 4K
+                                      // (profiles/r02_ab_gradient_geometry.txt): 16-block tiles in eight 4-warp CTAs per SM 130.1 us, 32-block tiles in
+                                      // four 8-warp CTAs 133.0 us — same resident warps, half as many warps behind each of the two CTA barriers
+#endif
+constexpr int PT_NB = J2P_TILE_BLOCKS;   // k_project_tile: CTA tile of PT_NB x 1 blocks
+constexpr int P22_NB = 16;               // k_project_tile22: CTA tile of 16 x 1 blocks
+constexpr int TP_NB = 4;                 // k_project_tma: warp tile of 4 x 1 blocks (8 lanes per block)
 
 // the stepped point at one frame pixel: y = x + f (x - xp), then y - step * (g / norm)
 // (compute.c:436, :213).  `rn` = RN(1/norm) from k_gradient's last CTA.
 struct Stepper {
     float factor, step, norm, rn;
-    bool stepping;
+    bool stepping;      // compute.c:211: no step when the norm is zero
+    bool norm_ok;       // the norm is a divisor the shared-reciprocal division is proven for
+    __device__ __forceinline__ Stepper(float factor_, float step_, float norm_, float rn_)
+        : factor(factor_), step(step_), norm(norm_), rn(rn_), stepping(norm_ != 0.f), norm_ok(qdiv_divisor_ok(norm_)) {}
     // IEEE division (generic / fallback paths)
     __device__ __forceinline__ float operator()(float x, float xp, float g) const {
         float y = fadd(x, fmul(factor, fsub(x, xp)));
@@ -49,6 +68,55 @@ struct Stepper2 {
         return addm2(mul2(nstep, qdiv2(g, nnorm, rn)), y, one);
     }
 };
+
+// Prologue of a CTA that projects plane c: threads 0..63 stage q, q*q and RN(1/(q*q)) into
+// sq[0..191], warp 2 the norm of g and its reciprocal into snorm[0..1] (whole frame: what
+// k_gradient left; strips: the fold of every rank's sums).  The caller synchronises the CTA.
+__device__ __forceinline__ void stage_tables(const FrameDev &F, int c, float *sq, float *snorm, int tid) {
+    if (tid < 64) {
+        sq[tid] = F.q[c][tid];
+        sq[64 + tid] = F.qq[c][tid];
+        sq[128 + tid] = F.rqq[c][tid];
+    }
+    if (tid >= 64 && tid < 96) strip_norm(F, c, snorm, tid - 64);
+}
+
+// x_k, x_{k-1} and g of four adjacent frame pixels
+struct Px4 {
+    float4 x, xp, g;
+};
+
+// Stepped point of a footprint of ZH rows x ZW pixels into z; ld(sy, k) returns pixels 4k..4k+3
+// of footprint row sy.  The fast pass divides by the shared reciprocal; if the guard rejects a
+// numerator of the footprint, or the norm itself, the footprint is stepped again with IEEE division.
+template <int ZH, int ZW, class Load>
+__device__ __forceinline__ void step_footprint(const Stepper &st, float (&z)[ZH][ZW], Load ld) {
+    static_assert(ZW % 4 == 0, "whole float4 pieces");
+    constexpr int N4 = ZW / 4;
+    unsigned key = 0xffffffffu;
+#pragma unroll
+    for (int sy = 0; sy < ZH; sy++)
+#pragma unroll
+        for (int k = 0; k < N4; k++) {
+            const Px4 p = ld(sy, k);
+            z[sy][k * 4 + 0] = st.fast(p.x.x, p.xp.x, p.g.x, key);
+            z[sy][k * 4 + 1] = st.fast(p.x.y, p.xp.y, p.g.y, key);
+            z[sy][k * 4 + 2] = st.fast(p.x.z, p.xp.z, p.g.z, key);
+            z[sy][k * 4 + 3] = st.fast(p.x.w, p.xp.w, p.g.w, key);
+        }
+    if (st.stepping && !(st.norm_ok && key >= QDIV_KEY_MIN)) {     // outside the proven range: IEEE division
+#pragma unroll
+        for (int sy = 0; sy < ZH; sy++)
+#pragma unroll
+            for (int k = 0; k < N4; k++) {
+                const Px4 p = ld(sy, k);
+                z[sy][k * 4 + 0] = st(p.x.x, p.xp.x, p.g.x);
+                z[sy][k * 4 + 1] = st(p.x.y, p.xp.y, p.g.y);
+                z[sy][k * 4 + 2] = st(p.x.z, p.xp.z, p.g.z);
+                z[sy][k * 4 + 3] = st(p.x.w, p.xp.w, p.g.w);
+            }
+    }
+}
 
 // (float)d for |d| < 2^22 without the conversion pipe (XU, a quarter of the fp32 rate and the busiest
 // pipe of the projection): 1.5 * 2^23 + d is exact as an integer add on the bit pattern, and
@@ -146,5 +214,64 @@ __device__ __forceinline__ void idct8x8_rows_x2(float (&a)[8], float (&b)[8], fl
     idct8(b);
 }
 
+// Clamp of row j of a block's DCT coefficients v to the quantisation interval (compute.c:323-331)
+// and the DCT-distance residual r = (t - d q) / (q q) (compute.c:47-49), num = t - d q.  draw: the
+// eight int16 coefficients of the row; sq: q, q*q, RN(1/(q*q)) as three rows of 64 (stage_tables).
+__device__ __forceinline__ void clamp_residual(float (&v)[8], float (&r)[8], float (&num)[8], int4 draw, const float *sq, int j) {
+    const int dw[4] = {draw.x, draw.y, draw.z, draw.w};
+    const float4 *t0 = reinterpret_cast<const float4 *>(&sq[j * 8]);
+    const float4 *t1 = reinterpret_cast<const float4 *>(&sq[64 + j * 8]);
+    const float4 *t2 = reinterpret_cast<const float4 *>(&sq[128 + j * 8]);
+    float qv[8], qqv[8], rqv[8];
+#pragma unroll
+    for (int k = 0; k < 2; k++) {
+        const float4 a = t0[k], bq = t1[k], cq = t2[k];
+        qv[k * 4] = a.x; qv[k * 4 + 1] = a.y; qv[k * 4 + 2] = a.z; qv[k * 4 + 3] = a.w;
+        qqv[k * 4] = bq.x; qqv[k * 4 + 1] = bq.y; qqv[k * 4 + 2] = bq.z; qqv[k * 4 + 3] = bq.w;
+        rqv[k * 4] = cq.x; rqv[k * 4 + 1] = cq.y; rqv[k * 4 + 2] = cq.z; rqv[k * 4 + 3] = cq.w;
+    }
+    unsigned rkey = 0xffffffffu;
+#pragma unroll
+    for (int i = 0; i < 8; i++) {
+        const int di = (i & 1) ? (dw[i >> 1] >> 16) : (int)(short)(dw[i >> 1] & 0xffff);
+        const float d = (float)di;
+        const float q = qv[i];
+        const float lo = fmul(fsub(d, 0.5f), q), hi = fmul(fadd(d, 0.5f), q);
+        float t = v[i];
+        t = t > hi ? hi : (t < lo ? lo : t);
+        v[i] = t;
+        num[i] = fsub(t, fmul(d, q));
+        rkey = min(rkey, qdiv_key(num[i]));
+        r[i] = qdiv_core(num[i], qqv[i], rqv[i]);                      // q*q in [1, 2^32] is always a valid divisor
+    }
+    if (rkey < QDIV_KEY_MIN) {                                       // a residual below 2^-60: IEEE division
+#pragma unroll
+        for (int i = 0; i < 8; i++) r[i] = fdiv(num[i], qqv[i]);
+    }
+}
+
+// Strips over peer memory, tile kernels: a CTA whose tile holds the strip's first / last two rows
+// also stores them into the neighbours' halo rows (NVLink stores), and the last border CTA of the
+// iteration raises their flag.  BP: frame pixels per side of a coefficient block (square sampling),
+// so the tile is BP rows high and starts at column bx0 * BP; it has C4 float4 pieces per row, of
+// which valid_c4 exist, and piece(row, c4) reads one from the (swizzled) staging of x_{k+1}.
+template <int NT, int BP, int C4, class Piece>
+__device__ __forceinline__ void deliver_border_rows(const FrameDev &F, int c, int by, int W, int valid_c4, int bx0, Piece piece) {
+    const StripSync &S = F.sync;
+    if (S.nranks > 1 && S.fused_halo) {
+        const bool top = by == 0 && S.has_up, bottom = by == (int)gridDim.y - 1 && S.has_down;
+        if (top || bottom) {
+            for (int e = threadIdx.x; e < 4 * C4; e += NT) {           // 2 rows x C4 pieces, top then bottom
+                const int side = e / (2 * C4), r = (e / C4) & 1, c4 = e % C4;
+                if (c4 >= valid_c4 || !(side ? bottom : top)) continue;
+                const int row = side ? BP - 2 + r : r;
+                float *dst = (side ? S.down_dst[c] : S.up_dst[c]) + (size_t)r * W + (size_t)bx0 * BP + (size_t)c4 * 4;
+                *reinterpret_cast<float4 *>(dst) = piece(row, c4);
+            }
+            if (top) strip_border_done(S, 0);
+            if (bottom) strip_border_done(S, 1);
+        }
+    }
+}
 
 }  // namespace j2p

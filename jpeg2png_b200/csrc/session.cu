@@ -41,9 +41,7 @@ cudaError_t launch_fold_sums(const double *sums_by_rank, int nranks, int nc, flo
 cudaError_t launch_decode(const int16_t *data, const float *q_host, float *out, int cw, int ch, cudaStream_t s);
 cudaError_t launch_init_plane(const float *fdata, float *x, float *xp, int W, int H, int cw, int ch, int sw, int sh,
                               cudaStream_t s);
-bool project_tma_enabled();
-int project_tma_border_units(const PlaneDev &P);
-int project_tile_border_units(const PlaneDev &P);
+int project_border_units(const FrameDev &F, int c);
 cudaError_t launch_scanlines(const float *Y, const float *Cb, const float *Cr, int W, int w, int h, int bits, uint8_t *out, cudaStream_t s);
 // kernels_strip.cu: the strip exchanges over peer memory (parameter blocks in kernels.cuh)
 cudaError_t launch_halo_exchange(const HaloPeers &P, unsigned seq, unsigned *ticket, int *err, int wait_for_arrival, cudaStream_t s);
@@ -1083,19 +1081,14 @@ static int p2p_bind(j2p_comm *c, j2p_session *s, const NcclApi *api) {
     if (ok) {
         s->ipc_exported = true;
         // Can the projection kernels deliver the border rows themselves?  Needs every plane to span
-        // the frame width (no stepped-only columns at the strip borders) and to go through one of
-        // the two tiled projection kernels (1x1 or 2x2 sampling).  The same on every rank: it only
-        // depends on the frame description.
+        // the frame width (no stepped-only columns at the strip borders) and to go through a kernel
+        // that delivers them.  The same on every rank: it only depends on the frame description.
         bool fused = true;
         unsigned ctas = 0;
         for (int k = 0; k < F.nc; k++) {
-            const PlaneDev &P = F.pl[k];
-            const bool tiled = (P.sw == 1 && P.sh == 1) || (P.sw == 2 && P.sh == 2);
-            fused = fused && tiled && P.cw * P.sw == F.W;
-            // units of work per block row that deliver border rows: warp tiles of the TMA kernel, CTA tiles of the cp.async kernels
-            if (P.sw == 1 && F.host_maps && project_tma_enabled()) ctas += (unsigned)project_tma_border_units(P);
-            else if (P.sw == 1) ctas += (unsigned)project_tile_border_units(P);
-            else ctas += (unsigned)(((P.cw >> 3) + 15) / 16);                     // kernels_project_tile22.cu: 16 blocks per CTA tile
+            const int units = project_border_units(F, k);
+            fused = fused && units > 0 && F.pl[k].cw * F.pl[k].sw == F.W;
+            ctas += (unsigned)units;
         }
         const char *e = getenv("J2P_STRIP_FUSED_HALO");
         if (e && *e == '0') fused = false;
@@ -1212,8 +1205,8 @@ extern "C" int j2p_session_iterate_strip(j2p_session *s, j2p_comm *c, unsigned n
     FrameDev &F = s->F;
     int rc;
     static const bool want_p2p = [] {
-        const char *e = getenv("J2P_STRIP_P2P"), *g = getenv("J2P_GRAD_SCALAR");
-        return !(e && *e == '0') && !(g && *g == '1');                   // the in-kernel exchanges live in the packed gradient kernel
+        const char *e = getenv("J2P_STRIP_P2P");
+        return !(e && *e == '0');
     }();
     if (want_p2p && c->p2p_state == 0 && (rc = p2p_bind(c, s, api)) != J2P_OK) return rc;
     const bool p2p = want_p2p && c->p2p_state == 1 && c->bound == s;

@@ -8,7 +8,9 @@ Three drivers of the same iteration are covered:
              happen inside the two solver kernels over NVLink, cudaIpc mappings
   nccl       the same entry point with J2P_STRIP_P2P=0: NCCL launches between the kernels
   unfused    peer memory, but the border rows travel in the stand-alone halo kernel
-             (J2P_STRIP_FUSED_HALO=0; what frames with uncovered columns use)"""
+             (J2P_STRIP_FUSED_HALO=0; what frames with uncovered columns use)
+  tma        peer memory with the luma plane projected by the TMA kernel (J2P_PROJ_TMA=1), whose
+             warp tiles deliver the fused border rows"""
 import os
 import tempfile
 
@@ -24,7 +26,8 @@ CASES = {
     # luma 1928 wide in a 1936-wide frame: stepped-only columns at the strip borders -> stand-alone halo kernel
     'uncovered': dict(w=1928, h=256, q=30, ss='4:2:0', weight=0.3, pw=[0.001] * 3, iters=12, tile=None),
 }
-MODES = {'torchdist': {}, 'native': {}, 'nccl': {'J2P_STRIP_P2P': '0'}, 'unfused': {'J2P_STRIP_FUSED_HALO': '0'}}
+MODES = {'torchdist': {}, 'native': {}, 'nccl': {'J2P_STRIP_P2P': '0'}, 'unfused': {'J2P_STRIP_FUSED_HALO': '0'},
+         'tma': {'J2P_PROJ_TMA': '1'}}
 
 
 def _frame(case):
@@ -92,7 +95,7 @@ def _run(world, mode, case, tmp_path, iters_check=None):
     H.assert_bit_identical(got, want, f'{world} strips ({mode}) vs {checker}')
 
 
-@pytest.mark.parametrize('mode', ['torchdist', 'native', 'nccl', 'unfused'])
+@pytest.mark.parametrize('mode', list(MODES))
 @pytest.mark.parametrize('world', [2, 4, 8])
 def test_strips_match_reference(world, mode, tmp_path):
     _run(world, mode, CASES['c420'], tmp_path)
